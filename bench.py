@@ -50,6 +50,7 @@ B_BITMAP = 1.0 / 8   # emitted set: one bit per record (this layout; SURVEY assu
 B_EXC = 4            # per record whose action is not the bare SUBMIT_HC: (offset << 8 | action)
 B_STOP = 12          # flags + finishedAt written when "Stopped" is first reported
 CONFIG_SEED = {2: 2, 3: 3, 5: 5}
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much in all
 WORKLOAD = {
     2: "BASELINE configs[1]: {n} HealthChecks per GPU, mixed 5-field cron + repeatAfterSec (tools/amgen config 2, "
        "seed 2); step = the single tick T0=2026-09-21T09:15:00Z",
@@ -178,6 +179,24 @@ def cpu_sweep_times(cols, T0, reps, threads, oracle_c, seconds=None):
     return times
 
 
+def write_outputs(out_dir, stats, idx=None, act=None):
+    """--dump-outputs: the last timed step's outputs as out_dir/<name>.npy.  stats.npy holds the tick's
+    statistics in STAT_FIELDS order (float64); due_index.npy / due_action.npy its due list (float64 /
+    float32, exact for these values).  A list too long for DUMP_BYTES is cut to a fixed, seeded sample of
+    its entries, kept in list order, so that two runs with the same arguments write the same files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "stats.npy"), np.asarray(stats, dtype=np.float64))
+    if idx is None:
+        return
+    room = (DUMP_BYTES - 4096) // 12  # 8 B index + 4 B action per entry; 4 KB for stats.npy and the headers
+    if len(idx) > room:
+        keep = np.sort(np.random.default_rng(0).choice(len(idx), room, replace=False))
+        idx, act = idx[keep], act[keep]
+    np.save(os.path.join(out_dir, "due_index.npy"), np.asarray(idx, dtype=np.float64))
+    np.save(os.path.join(out_dir, "due_action.npy"), np.asarray(act, dtype=np.float32))
+
+
 def run_reference(args, rank, world):
     """--impl reference: the CPU path on this box's host cores.  The reference is Go
     (robfig/cron un-vendored, no Go toolchain): this times oracle/ — our C restatement of the
@@ -204,9 +223,12 @@ def run_reference(args, rank, world):
     t0 = time.perf_counter()
     for k in range(args.steps):
         t1 = time.perf_counter()
-        oracle_c.sweep(work, T0, threads=threads, buffers=bufs)
+        last = oracle_c.sweep(work, T0, threads=threads, buffers=bufs)
         times.append(time.perf_counter() - t1)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        idx, act, st = last
+        write_outputs(args.dump_outputs, [st[f] for f in oracle_c.STAT_FIELDS], idx, act)
     value = n * args.steps / dt
     sample = f"{n} records x {args.steps} ticks (whole config-2 population of the N={world} run each step)"
     print(json.dumps({
@@ -248,12 +270,21 @@ def main():
                          "plain list push, or the padded NCCL all-gather")
     ap.add_argument("--settle-ms", type=float, default=400.0,
                     help="untimed load before the warm-up steps so SM clocks settle (reported as settle_steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB): "
+                         "stats.npy (the tick's statistics) and, except for --config 5, whose step returns statistics "
+                         "only, due_index.npy / due_action.npy (the tick's due list).  Inputs are seeded, so two "
+                         "builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and args.impl == "ours" and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one GPU: run it with --gpus 1")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -392,6 +423,11 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    def last_list():
+        """host copies of what the last tick_device step left on the device: (stats, due list, actions)"""
+        cnt = int(d_cnt.item())
+        return d_st.cpu().numpy(), d_idx[:cnt].cpu().numpy(), d_act[:cnt].cpu().numpy()
+
     # ---- N>1: is the gathered list right?  checked before and after the timed loop ----
     verify = None
 
@@ -457,6 +493,7 @@ def main():
         w0 = time.perf_counter()
         stats_k = sweep.run_ticks(T0 + settle, args.steps, am.SWEEP_CLOSED_LOOP, seed)
         wall = time.perf_counter() - w0
+        last = ([stats_k[f][-1] for f in am.abi.STAT_FIELDS],)
         ms = sweep.last_kernel_ms
         launches = sweep.launch_count - launches0
         sweep.run_ticks(T0 + settle + args.steps, max(64, int(800 / 0.1)), am.SWEEP_CLOSED_LOOP, seed)
@@ -499,6 +536,7 @@ def main():
             step(k)
             evs[k][1].record(stream)
         torch.cuda.synchronize()
+        last = last_list() if args.dump_outputs else None
         per_step_ms = [a.elapsed_time(b) for a, b in evs]
         ms = sum(per_step_ms)
         launches = sweep.launch_count - launches0
@@ -551,6 +589,7 @@ def main():
         drain()
         ev1.record(stream)
         barrier()
+        last = last_list() if args.dump_outputs else None
         ms = ev0.elapsed_time(ev1)
         launches = sweep.launch_count - launches0 + gather_launches[0] - gl0
         if world > 1:
@@ -812,6 +851,8 @@ def main():
             out.update(verify)
         if config == 5 and blocking is not None:
             out["temporal_blocking"] = blocking
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, *last)
         print(json.dumps(out))
     if world > 1:
         dist.barrier()

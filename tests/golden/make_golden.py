@@ -5,6 +5,11 @@ NOT outputs of the reference: they are outputs of the C oracle, accepted only
 when the independent Python oracle reproduces them, frozen so that later edits
 to either oracle or to the kernel are checked against a fixed point.
 Re-run:  python tests/golden/make_golden.py
+
+examples/healthchecks.json holds the HealthCheck manifests of active-monitor's
+examples/ directory (Apache-2.0), converted from YAML to JSON and keyed by their
+path there, so that the ingest tests need no checkout of that project.
+Re-run:  python tests/golden/make_golden.py --examples <active-monitor>/examples
 """
 import hashlib
 import json
@@ -67,5 +72,23 @@ def main():
         print(name, "ok", [t["stats"]["n_emitted"] for t in out["ticks"]][:6])
 
 
+def examples(src):
+    import glob
+    import yaml
+    docs = {}
+    for path in sorted(glob.glob(os.path.join(src, "**", "*.yaml"), recursive=True)):
+        for doc in yaml.safe_load_all(open(path)):
+            if isinstance(doc, dict) and doc.get("kind") == "HealthCheck":
+                docs[os.path.relpath(path, src)] = doc
+    os.makedirs(os.path.join(HERE, "examples"), exist_ok=True)
+    with open(os.path.join(HERE, "examples", "healthchecks.json"), "w") as f:
+        json.dump(docs, f, indent=1, ensure_ascii=False)
+        f.write("\n")
+    print("examples ok", len(docs))
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["--examples"]:
+        examples(sys.argv[2])
+    else:
+        main()

@@ -1,24 +1,18 @@
 """The reference's own example / BDD manifests through the product's ladder
-(SURVEY.md section 8f-2).  Reads /root/reference, so it only runs where the reference
-tree is mounted (never on the GPU box; not a gpu test)."""
-import glob
+(SURVEY.md section 8f-2).  The manifests are stored as JSON in
+tests/golden/examples/healthchecks.json, keyed by their path under the reference's examples/."""
 import importlib
+import json
 import os
 
-import pytest
-import yaml
+from conftest import ROOT
 
-REF = "/root/reference/examples"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
+EXAMPLES = os.path.join(ROOT, "tests", "golden", "examples", "healthchecks.json")
 
 
 def _docs():
-    out = {}
-    for path in sorted(glob.glob(os.path.join(REF, "**", "*.yaml"), recursive=True)):
-        for doc in yaml.safe_load_all(open(path)):
-            if isinstance(doc, dict) and doc.get("kind") == "HealthCheck":
-                out[os.path.relpath(path, REF)] = doc
-    return out
+    with open(EXAMPLES, encoding="utf-8") as f:
+        return json.load(f)
 
 
 def test_every_example_classifies(am):

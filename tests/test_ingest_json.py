@@ -1,7 +1,6 @@
 """Native manifest ingest (am_healthcheck_ingest_json, SURVEY 8f-2): JSON as the API server serves it ->
 packed records, against (a) the ORACLE's ladder fed by an independent Python reading of the same documents
 (json.loads + the field names of healthcheck_types.go) and (b) the reference's example / BDD manifests."""
-import glob
 import importlib
 import json
 import os
@@ -9,6 +8,8 @@ import random
 
 import numpy as np
 import pytest
+
+from conftest import ROOT
 
 ingest = importlib.import_module("active-monitor_b200.ingest")
 am = importlib.import_module("active-monitor_b200")
@@ -108,17 +109,9 @@ def test_restart_semantics_and_errors():
     assert len(recs) == 0
 
 
-REF = "/root/reference/examples"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 def test_reference_examples_through_the_native_ingest():
-    import yaml
-    docs = []
-    for path in sorted(glob.glob(os.path.join(REF, "**", "*.yaml"), recursive=True)):
-        for doc in yaml.safe_load_all(open(path)):
-            if isinstance(doc, dict) and doc.get("kind") == "HealthCheck":
-                docs.append(doc)
+    with open(os.path.join(ROOT, "tests", "golden", "examples", "healthchecks.json"), encoding="utf-8") as f:
+        docs = list(json.load(f).values())
     assert len(docs) >= 12
     rcs, recs = ingest.ingest_json(json.dumps({"kind": "List", "items": docs}))
     for i, doc in enumerate(docs):
