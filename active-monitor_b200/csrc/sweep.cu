@@ -30,6 +30,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -126,8 +127,6 @@ struct am_sweep {
   uint64_t capacity = 0, cap_padded = 0, shard_base = 0;
   uint64_t n_records = 0;  // high-water mark
   DevCols cols{};
-  void* col_ptr[16] = {};
-  size_t col_elem[16] = {};
   TickSet set[2];
   uint32_t parity = 0;
   int last_shard_parity = -1;
@@ -187,27 +186,11 @@ namespace {
     }                                                                                 \
   } while (0)
 
-constexpr size_t kColElem[16] = {8, 8, 8, 8, 8, 4, 4, 8, 4, 4, 4, 4, 4, 4, 4, 8};
-
-void** col_slot(DevCols& c, int k) {
-  void** slots[16] = {(void**)&c.minute,         (void**)&c.hour,          (void**)&c.dom,
-                      (void**)&c.month,          (void**)&c.dow,           (void**)&c.ras,
-                      (void**)&c.flags,          (void**)&c.finished_at,   (void**)&c.runs_limit,
-                      (void**)&c.reset_interval, (void**)&c.success,       (void**)&c.failed,
-                      (void**)&c.remedy_success, (void**)&c.remedy_failed, (void**)&c.remedy_total,
-                      (void**)&c.remedy_finished_at};
-  return slots[k];
-}
-void* const* cols_member(const am_record_cols_t* c, int k) {
-  void* const* slots[16] = {(void* const*)&c->minute,         (void* const*)&c->hour,
-                            (void* const*)&c->dom,            (void* const*)&c->month,
-                            (void* const*)&c->dow,            (void* const*)&c->ras,
-                            (void* const*)&c->flags,          (void* const*)&c->finished_at,
-                            (void* const*)&c->runs_limit,     (void* const*)&c->reset_interval,
-                            (void* const*)&c->success,        (void* const*)&c->failed,
-                            (void* const*)&c->remedy_success, (void* const*)&c->remedy_failed,
-                            (void* const*)&c->remedy_total,   (void* const*)&c->remedy_finished_at};
-  return slots[k];
+// Column k (0..15, AM_RECORD_COLUMNS order) of a column set, untyped; its element size is kColumns[k].elem.
+template <typename Cols>  // am_record_cols_t or const am_record_cols_t
+auto& column(Cols& c, int k) {
+  using Ptr = typename std::conditional<std::is_const<Cols>::value, void* const, void*>::type;
+  return reinterpret_cast<Ptr*>(&c)[k];
 }
 
 struct TickGuard {
@@ -679,13 +662,10 @@ int am_sweep_create(am_sweep_t** out, int device_id, uint64_t capacity, uint64_t
       AM_CUDA(h, cudaEventCreateWithFlags(&h->stage[b].drained, cudaEventDisableTiming));
       AM_CUDA(h, cudaEventCreateWithFlags(&h->set[b].consumed, cudaEventDisableTiming));
     }
-    for (int k = 0; k < 16; ++k) {
-      void* p = nullptr;
-      AM_CUDA(h, cudaMalloc(&p, h->cap_padded * kColElem[k]));
-      AM_CUDA(h, cudaMemsetAsync(p, 0, h->cap_padded * kColElem[k], h->stream));
-      *col_slot(h->cols, k) = p;
-      h->col_ptr[k] = p;
-      h->col_elem[k] = kColElem[k];
+    for (int k = 0; k < kNumCols; ++k) {
+      void*& p = column(h->cols, k);
+      AM_CUDA(h, cudaMalloc(&p, h->cap_padded * kColumns[k].elem));
+      AM_CUDA(h, cudaMemsetAsync(p, 0, h->cap_padded * kColumns[k].elem, h->stream));
     }
     AM_LAUNCH(fill_u32_kernel, 1184, 256, h->stream, h->cols.flags, AM_F_TOMBSTONE, h->cap_padded);
     h->launches++;
@@ -733,7 +713,7 @@ void am_sweep_destroy(am_sweep_t* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();  // ticks may have been issued on caller streams
-  for (int k = 0; k < 16; ++k) if (h->col_ptr[k]) cudaFree(h->col_ptr[k]);
+  for (int k = 0; k < kNumCols; ++k) if (column(h->cols, k)) cudaFree(column(h->cols, k));
   for (int b = 0; b < 2; ++b) {
     TickOut& t = h->set[b].out;
     if (t.bitmap) cudaFree(t.bitmap);
@@ -771,8 +751,8 @@ uint64_t am_sweep_capacity(const am_sweep_t* h) { return h ? h->capacity : 0; }
 int am_sweep_device(const am_sweep_t* h) { return h ? h->device : -1; }
 double am_sweep_last_kernel_ms(const am_sweep_t* h) { return h ? h->last_ms : -1.0; }
 uint64_t am_sweep_launch_count(const am_sweep_t* h) { return h ? h->launches : 0; }
-void* am_sweep_column_ptr(am_sweep_t* h, int column) {
-  return (h && column >= 0 && column < 16) ? h->col_ptr[column] : nullptr;
+void* am_sweep_column_ptr(am_sweep_t* h, int id) {
+  return (h && id >= 0 && id < kNumCols) ? column(h->cols, id) : nullptr;
 }
 int am_sweep_set_profiling(am_sweep_t* h, int on) {
   if (!h) return AM_E_INVAL;
@@ -806,11 +786,12 @@ int am_sweep_load_range(am_sweep_t* h, uint64_t first, uint64_t n, const am_reco
   AM_CUDA(h, cudaSetDevice(h->device));
   int rc = order_on(h, h->stream);
   if (rc != AM_OK) return rc;
-  for (int k = 0; k < 16; ++k) {
-    char* dst = (char*)h->col_ptr[k] + first * kColElem[k];
-    const void* src = *cols_member(cols, k);
-    if (src) AM_CUDA(h, cudaMemcpyAsync(dst, src, n * kColElem[k], cudaMemcpyHostToDevice, h->stream));
-    else AM_CUDA(h, cudaMemsetAsync(dst, 0, n * kColElem[k], h->stream));
+  for (int k = 0; k < kNumCols; ++k) {
+    const size_t elem = kColumns[k].elem;
+    char* dst = (char*)column(h->cols, k) + first * elem;
+    const void* src = column(*cols, k);
+    if (src) AM_CUDA(h, cudaMemcpyAsync(dst, src, n * elem, cudaMemcpyHostToDevice, h->stream));
+    else AM_CUDA(h, cudaMemsetAsync(dst, 0, n * elem, h->stream));
   }
   AM_CUDA(h, cudaStreamSynchronize(h->stream));
   if (first + n > h->n_records) h->n_records = first + n;
@@ -1177,11 +1158,11 @@ int am_sweep_read(am_sweep_t* h, uint64_t first, uint64_t n, const uint64_t* idx
 static int read_impl(am_sweep_t* h, uint64_t first, uint64_t n, const uint64_t* idx, am_record_cols_t* out) {
   if (!idx) {
     if (first + n > h->capacity || first + n < first) return AM_E_INVAL;
-    for (int k = 0; k < 16; ++k) {
-      void* dst = *cols_member(out, k);
+    for (int k = 0; k < kNumCols; ++k) {
+      void* dst = column(*out, k);
       if (!dst) continue;
-      AM_CUDA(h, cudaMemcpyAsync(dst, (char*)h->col_ptr[k] + first * kColElem[k], n * kColElem[k],
-                                 cudaMemcpyDeviceToHost, h->stream));
+      const size_t elem = kColumns[k].elem;
+      AM_CUDA(h, cudaMemcpyAsync(dst, (char*)column(h->cols, k) + first * elem, n * elem, cudaMemcpyDeviceToHost, h->stream));
     }
     AM_CUDA(h, cudaStreamSynchronize(h->stream));
     return AM_OK;
@@ -1203,24 +1184,11 @@ static int read_impl(am_sweep_t* h, uint64_t first, uint64_t n, const uint64_t* 
   AM_CUDA(h, cudaMemcpyAsync(h->pin_in.p, dp, n * sizeof(am_record_t), cudaMemcpyDeviceToHost, h->stream));
   AM_CUDA(h, cudaStreamSynchronize(h->stream));
   const am_record_t* r = (const am_record_t*)h->pin_in.p;
-  for (uint64_t k = 0; k < n; ++k) {
-    if (out->minute) out->minute[k] = r[k].minute;
-    if (out->hour) out->hour[k] = r[k].hour;
-    if (out->dom) out->dom[k] = r[k].dom;
-    if (out->month) out->month[k] = r[k].month;
-    if (out->dow) out->dow[k] = r[k].dow;
-    if (out->ras) out->ras[k] = r[k].ras;
-    if (out->flags) out->flags[k] = r[k].flags;
-    if (out->finished_at) out->finished_at[k] = r[k].finished_at;
-    if (out->runs_limit) out->runs_limit[k] = r[k].runs_limit;
-    if (out->reset_interval) out->reset_interval[k] = r[k].reset_interval;
-    if (out->success) out->success[k] = r[k].success;
-    if (out->failed) out->failed[k] = r[k].failed;
-    if (out->remedy_success) out->remedy_success[k] = r[k].remedy_success;
-    if (out->remedy_failed) out->remedy_failed[k] = r[k].remedy_failed;
-    if (out->remedy_total) out->remedy_total[k] = r[k].remedy_total;
-    if (out->remedy_finished_at) out->remedy_finished_at[k] = r[k].remedy_finished_at;
-  }
+#define AM_SCATTER(name) \
+  if (out->name)         \
+    for (uint64_t k = 0; k < n; ++k) out->name[k] = r[k].name;
+  AM_RECORD_COLUMNS(AM_SCATTER)
+#undef AM_SCATTER
   return AM_OK;
 }
 

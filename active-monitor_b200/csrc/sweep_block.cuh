@@ -17,7 +17,8 @@
 //   posted result / carry bits  the first tick of the block
 //
 // and at an event tick evaluates EXACTLY what sweep_tick_kernel evaluates for that (record, tick) —
-// same ladder, same apply_result, same closed-loop outcome key — so the per-tick statistics and the
+// the same ladder, and the same helpers of sweep_kernels.cuh for the rest: evaluated, apply_result,
+// complete_closed_loop — so the per-tick statistics and the
 // columns after the block are bit-identical to K single ticks (tests: run_ticks blocked == unblocked ==
 // oracle).  Work is O(events), not O(records x ticks); the columns are read and written once per K
 // ticks.  What it does NOT produce is the per-tick (index, action) lists: a run of ticks publishes
@@ -27,22 +28,14 @@
 
 namespace amsweep {
 
-#ifndef AM_BLOCK_MAX_TICKS
-#define AM_BLOCK_MAX_TICKS 128
-#endif
-constexpr int kMaxBlockTicks = AM_BLOCK_MAX_TICKS;
+constexpr int kMaxBlockTicks = 128;
 constexpr int kDefaultBlockTicks = 96;  // 16.0 us per tick; 64: 18.1, 128: 17.3 (tools/r02_run17.sh, 10 M records, config 5)
-#ifndef AM_BLOCK_THREADS
-#define AM_BLOCK_THREADS 128
-#endif
-constexpr int kBlockThreads = AM_BLOCK_THREADS;
+constexpr int kBlockThreads = 128;
 // Occupancy is what this kernel wants: its warps wait on each other (per-class lists of different lengths, one
 // barrier before the flush) and on shared atomics.  256 threads at 94 registers = 2 CTAs per SM: 27.3 us per tick,
 // 52 % of the stall samples at the final barrier.  128 threads: 23.2.  128 threads capped at 64 registers (8 CTAs per
 // SM, 4 bytes of spills): 18.0; the same at 256 threads / 4 CTAs: 16.8.  (tools/r02_run15.sh .. r02_run17.sh)
-#ifndef AM_BLOCK_MIN_CTAS
-#define AM_BLOCK_MIN_CTAS 8
-#endif
+constexpr int kBlockMinCtas = 8;
 constexpr int kBlockRecords = 4 * kBlockThreads;  // four consecutive records per thread in the classification pass
 constexpr int kBlockClasses = 4;                  // by expected number of events in the block: <= 2, <= 8, <= 24, more
 
@@ -160,14 +153,7 @@ __device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S
       s.flags = f;
       s.fa = fa;
       uint32_t a = apply_result(s, T, res);
-      if (CLOSED && due) {
-        const uint64_t key = outcome_key(p.seed, g, (uint64_t)T);
-        const uint32_t failp = (s.flags >> AM_F_FAILP_SHIFT) & 0xFFu;
-        const bool fail = (uint32_t)(key & 0xFF) < failp;
-        const bool rem_ok = (uint32_t)((key >> 8) & 0xFF) < 179u;
-        s.flags |= (fail ? AM_F_PENDING_FAIL : AM_F_PENDING_OK) | AM_F_REMEDY_PENDING | (rem_ok ? AM_F_REMEDY_OUTCOME_OK : 0u);
-        a |= apply_result(s, T, res);
-      }
+      if (CLOSED && due) a |= complete_closed_loop(s, p.seed, g, T, res);
       act |= a;
       f = s.flags;
       fa = s.fa;
@@ -210,7 +196,7 @@ __device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S
 }
 
 template <bool CLOSED>
-__global__ void __launch_bounds__(kBlockThreads, AM_BLOCK_MIN_CTAS) sweep_block_kernel(const BlockParams p) {
+__global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kernel(const BlockParams p) {
   __shared__ BlockStats S;
   const int tid = threadIdx.x;
   {
@@ -245,8 +231,7 @@ __global__ void __launch_bounds__(kBlockThreads, AM_BLOCK_MIN_CTAS) sweep_block_
       const int64_t fa = q == 0 ? a01.x : q == 1 ? a01.y : q == 2 ? a23.x : a23.y;
       const uint32_t loc = loc0 + (uint32_t)q;
       const uint32_t kind = f & AM_KIND_MASK;
-      const bool live = ((0x3Eu >> kind) & 1u) && !(f & AM_F_TOMBSTONE);
-      if (!live) continue;  // tombstones, NO_RESOURCE (hcc.go:227), host-fallback: never evaluated
+      if (!evaluated(f)) continue;
       const bool first_tick = (f & (kPend | AM_F_CARRY_MASK)) != 0;  // a posted result / carried action: an event at tick 0
       const uint64_t g = p.shard_base + cta_base + loc;
       int64_t n_ev = 0;  // expected events in the block (an upper bound is fine: it only picks the list)

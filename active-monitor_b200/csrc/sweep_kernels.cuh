@@ -195,6 +195,37 @@ __device__ __forceinline__ uint32_t carry_of_actions(uint32_t a) { return ((a & 
 static_assert(AM_F_CARRY_SHIFT == 11 && AM_ACT_RUN_REMEDY == 0x02u && AM_ACT_REMEDY_SKIP == 0x10u && AM_ACT_ANOMALY == 0x80u,
               "carry bit layout");
 
+// Is the record evaluated at all: kinds 1..5 are; tombstones, NO_RESOURCE (hcc.go:227) and host-fallback are not.
+// (The sweep expands the macro in place, on the kind it has already extracted: only then does the compiler fold it
+// into the kind tests of the ladder — through the function, sweep_tick_kernel<1,0> issues 8 more instructions.)
+#define AM_EVALUATED(f, kind) (((0x3Eu >> (kind)) & 1u) && !((f) & AM_F_TOMBSTONE))
+__device__ __forceinline__ bool evaluated(uint32_t f) { return AM_EVALUATED(f, f & AM_KIND_MASK); }
+
+// Closed-loop harness (config 5, DESIGN §6.7): a due record completes in the same tick with its preset
+// outcome — failed iff key byte 0 < the record's failp8, remedy succeeded iff key byte 1 < kRemedyOkBelow
+// — taken like a posted result (hcc.go:635-724).  Returns the action bits of that result.
+constexpr uint32_t kRemedyOkBelow = 179;  // of 256: a remedy succeeds 70 % of the time
+__device__ __forceinline__ uint32_t complete_closed_loop(RecState& s, uint64_t seed, uint64_t gidx, int64_t T, uint32_t& res) {
+  const uint64_t k = outcome_key(seed, gidx, (uint64_t)T);
+  const uint32_t failp = (s.flags >> AM_F_FAILP_SHIFT) & 0xFFu;
+  const bool fail = (uint32_t)(k & 0xFF) < failp;
+  const bool rem_ok = (uint32_t)((k >> 8) & 0xFF) < kRemedyOkBelow;
+  s.flags |= (fail ? AM_F_PENDING_FAIL : AM_F_PENDING_OK) | AM_F_REMEDY_PENDING | (rem_ok ? AM_F_REMEDY_OUTCOME_OK : 0u);
+  return apply_result(s, T, res);
+}
+
+// Results applied (metrics.MonitorSuccess / Error; hcc.go:635-722, :821-851): the four byte counters of
+// apply_result's `res` {ok, fail, remedy ok, remedy fail} summed over the warp (two redux over 16-bit halves).
+// Lane q < 4 receives counter q, the other lanes 0.
+__device__ __forceinline__ uint32_t warp_result_counts(uint32_t res, int lane) {
+  uint32_t lo = 0, hi = 0;
+  if (__any_sync(kFull, res != 0)) {
+    lo = __reduce_add_sync(kFull, (res & 0xFFu) | ((res & 0xFF00u) << 8));           // ok | fail<<16
+    hi = __reduce_add_sync(kFull, ((res >> 16) & 0xFFu) | ((res >> 8) & 0xFF0000u));  // remedy ok | fail<<16
+  }
+  return lane < 4 ? ((lane < 2 ? lo : hi) >> ((lane & 1) * 16)) & 0xFFFFu : 0u;
+}
+
 // robfig SpecSchedule matching against the tick's one-hot wall-clock words (Appendix A: five ANDs and
 // the dom/dow star rule).  Branch-free: every term is evaluated (no short-circuit control flow).
 __device__ __forceinline__ bool cron_matches(const TickWords& t, uint64_t mi, uint64_t hr, uint64_t dm, uint64_t mo, uint64_t dw) {
@@ -228,15 +259,13 @@ __global__ void tz_words_kernel(const int32_t* __restrict__ tz_off, TickWords* _
 // The sweep.  CLOSED = closed-loop harness (SURVEY §8d config 5): a due record
 // completes in the same tick with its preset outcome.
 // ---------------------------------------------------------------------------
-#ifndef AM_MIN_BLOCKS
-#define AM_MIN_BLOCKS 3
-#endif
+constexpr int kMinBlocks = 3;  // CTAs per SM with the mask columns; one more without them
 // MASKS = the five cron-field columns are read and matched.  Off the minute a
 // 5-field schedule cannot fire (ParseStandard pins Second to 1<<0), so the
 // launcher picks MASKS=false unless AM_SWEEP_FULL_SCAN is set: 40 of the 56
 // bytes per record and all of the mask arithmetic disappear at compile time.
 template <bool CLOSED, bool MASKS>
-__global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS + 1) sweep_tick_kernel(const SweepParams p) {
+__global__ void __launch_bounds__(kBlock, MASKS ? kMinBlocks : kMinBlocks + 1) sweep_tick_kernel(const SweepParams p) {
   // one row per warp, written unconditionally: no zero-initialisation, no shared
   // atomics, and therefore a single __syncthreads in the whole kernel
   __shared__ uint32_t s_warp_tot[kWarps], s_warp_exc[kWarps];
@@ -250,9 +279,6 @@ __global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS 
   const uint32_t tile_base = tile * (uint32_t)kTile;
   const int64_t T = p.T;
   pdl_wait();  // the sweep is launched while its predecessor (the previous tick's publish, or the drain) still runs
-#ifdef AM_SWEEP_TRIGGER
-  pdl_trigger();  // (A/B) scan_groups_kernel may become resident during the sweep's tail
-#endif
 
   // ---- phase A: issue every schedule-column load of this lane up front ----
   // half h covers records r0(h) .. r0(h)+1, r0 = tile_base + warp*128 + h*64 + lane*2
@@ -309,8 +335,7 @@ __global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS 
       const int32_t rasv = j ? ras[h].y : ras[h].x;
       const int64_t fav = j ? fa[h].y : fa[h].x;
       const uint32_t kind = f & AM_KIND_MASK;
-      // kinds 1..5 are evaluated; tombstones, NO_RESOURCE (hcc.go:227) and host-fallback are not
-      const bool live = ((0x3Eu >> kind) & 1u) && !(f & AM_F_TOMBSTONE);
+      const bool live = AM_EVALUATED(f, kind);
       const bool has_result = (f & (AM_F_PENDING_OK | AM_F_PENDING_FAIL)) != 0;
       const bool pending = (f & (AM_F_PENDING_OK | AM_F_PENDING_FAIL | AM_F_REMEDY_PENDING)) != 0;
       // step 1 sets finishedAt = T before the due decision is taken
@@ -419,15 +444,7 @@ __global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS 
             RecState s{nfl[h][j], nfa[h][j], ns[j], nf[j], nrs[j], nrf[j], nrt[j], nrfa[j], limv[j], rstv[j]};
             uint32_t res = 0;
             uint32_t a = apply_result(s, T, res);
-            if (CLOSED && ((due_bits >> (2 * h + j)) & 1u)) {
-              const uint64_t k = outcome_key(p.seed, p.shard_base + r + (uint32_t)j, (uint64_t)T);
-              const uint32_t failp = (s.flags >> AM_F_FAILP_SHIFT) & 0xFFu;
-              const bool fail = (uint32_t)(k & 0xFF) < failp;
-              const bool rem_ok = (uint32_t)((k >> 8) & 0xFF) < 179u;
-              s.flags |= (fail ? AM_F_PENDING_FAIL : AM_F_PENDING_OK) | AM_F_REMEDY_PENDING |
-                         (rem_ok ? AM_F_REMEDY_OUTCOME_OK : 0u);
-              a |= apply_result(s, T, res);
-            }
+            if (CLOSED && ((due_bits >> (2 * h + j)) & 1u)) a |= complete_closed_loop(s, p.seed, p.shard_base + r + (uint32_t)j, T, res);
             act[h][j] |= a;
             res_lane += res;
             nfl[h][j] = s.flags; nfa[h][j] = s.fa;
@@ -464,15 +481,7 @@ __global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS 
       RecState s{f0, fa0, sc, fc, rsc, rfc, rtc, rfa, lim, rst};
       uint32_t res = 0;
       uint32_t a = apply_result(s, T, res);
-      if (CLOSED && ((due_bits >> b) & 1u)) {
-        const uint64_t k = outcome_key(p.seed, p.shard_base + i, (uint64_t)T);
-        const uint32_t failp = (s.flags >> AM_F_FAILP_SHIFT) & 0xFFu;
-        const bool fail = (uint32_t)(k & 0xFF) < failp;
-        const bool rem_ok = (uint32_t)((k >> 8) & 0xFF) < 179u;
-        s.flags |= (fail ? AM_F_PENDING_FAIL : AM_F_PENDING_OK) | AM_F_REMEDY_PENDING |
-                   (rem_ok ? AM_F_REMEDY_OUTCOME_OK : 0u);
-        a |= apply_result(s, T, res);
-      }
+      if (CLOSED && ((due_bits >> b) & 1u)) a |= complete_closed_loop(s, p.seed, p.shard_base + i, T, res);
       res_lane += res;  // per lane at most 4 records x 2 results per byte
       if (s.s != sc) st_stream(p.c.success + i, s.s);
       if (s.f != fc) st_stream(p.c.failed + i, s.f);
@@ -525,12 +534,8 @@ __global__ void __launch_bounds__(kBlock, MASKS ? AM_MIN_BLOCKS : AM_MIN_BLOCKS 
   //      statistics and index checksums are derived from the emitted entries
   //      by expand_kernel, so records that emit nothing cost nothing here.
   {
-    uint32_t lo = 0, hi = 0;
-    if (__any_sync(kFull, res_lane != 0)) {
-      lo = __reduce_add_sync(kFull, (res_lane & 0xFFu) | ((res_lane & 0xFF00u) << 8));           // ok | fail<<16
-      hi = __reduce_add_sync(kFull, ((res_lane >> 16) & 0xFFu) | ((res_lane >> 8) & 0xFF0000u));  // remedy ok | fail<<16
-    }
-    if (lane < 4) s_wres[warp][lane] = ((lane < 2 ? lo : hi) >> ((lane & 1) * 16)) & 0xFFFFu;
+    const uint32_t v = warp_result_counts(res_lane, lane);
+    if (lane < 4) s_wres[warp][lane] = v;
   }
   __syncthreads();
 
@@ -899,7 +904,7 @@ __global__ void next_due_kernel(DevCols c, uint64_t n, int64_t T, unsigned long 
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
     const uint32_t f = c.flags[i];
     const uint32_t kind = f & AM_KIND_MASK;
-    if ((f & AM_F_TOMBSTONE) || !((0x3Eu >> kind) & 1u)) continue;
+    if (!evaluated(f)) continue;
     int64_t due = INT64_MAX;
     if ((f & (AM_F_PENDING_OK | AM_F_PENDING_FAIL | AM_F_REMEDY_PENDING)) || kind == AM_KIND_PARSE_ERROR ||
         (kind == AM_KIND_STOPPED && !(f & AM_F_STOPPED_REPORTED))) {
@@ -964,12 +969,9 @@ __global__ void apply_state_ops_kernel(DevCols c, const uint32_t* __restrict__ m
   if (kind == kOpResult || marks[3u * i] != k + 1u) return;
   if (kind == kOpRemove) { c.flags[i] = AM_F_TOMBSTONE; return; }
   const am_record_t r = recs[arg & ~kOpKindMask];
-  c.minute[i] = r.minute; c.hour[i] = r.hour; c.dom[i] = r.dom; c.month[i] = r.month; c.dow[i] = r.dow;
-  c.ras[i] = r.ras; c.flags[i] = r.flags; c.finished_at[i] = r.finished_at;
-  c.runs_limit[i] = r.runs_limit; c.reset_interval[i] = r.reset_interval;
-  c.success[i] = r.success; c.failed[i] = r.failed; c.remedy_success[i] = r.remedy_success;
-  c.remedy_failed[i] = r.remedy_failed; c.remedy_total[i] = r.remedy_total;
-  c.remedy_finished_at[i] = r.remedy_finished_at;
+#define AM_STORE(name) c.name[i] = r.name;
+  AM_RECORD_COLUMNS(AM_STORE)
+#undef AM_STORE
 }
 
 // terminal phases observed by the watch loops (hcc.go:635/:662/:821/:836).  The winner of
@@ -1026,8 +1028,7 @@ __global__ void apply_results_now_kernel(DevCols c, const uint32_t* __restrict__
       uint32_t f = c.flags[i];
       if (mine_hc) f = (f & ~kHcBits) | (arg & kHcBits);
       if (rm_valid) f = (f & ~kRemedyBits) | ((mine_rm ? arg : ops[rmw - 1u].y) & kRemedyBits);
-      const bool live = ((0x3Eu >> (f & AM_KIND_MASK)) & 1u) && !(f & AM_F_TOMBSTONE);
-      if (!live || !(f & kPend)) {
+      if (!evaluated(f) || !(f & kPend)) {
         c.flags[i] = f;  // (a record the sweep does not evaluate keeps its posted result)
       } else {
         // Gather only what this result can touch (every column is its own 32-B sector of a random record):
@@ -1060,16 +1061,10 @@ __global__ void apply_results_now_kernel(DevCols c, const uint32_t* __restrict__
       }
     }
   }
-  // results applied (metrics.MonitorSuccess / Error): warp -> global RED, as the sweep does per tile
-  if (__any_sync(kFull, res != 0)) {
-    const uint32_t lo = __reduce_add_sync(kFull, (res & 0xFFu) | ((res & 0xFF00u) << 8));
-    const uint32_t hi = __reduce_add_sync(kFull, ((res >> 16) & 0xFFu) | ((res >> 8) & 0xFF0000u));
-    const int lane = threadIdx.x & 31;
-    if (lane < 4) {
-      const uint32_t v = ((lane < 2 ? lo : hi) >> ((lane & 1) * 16)) & 0xFFFFu;
-      if (v) atomicAdd(&acc[10 + lane], (unsigned long long)v);
-    }
-  }
+  // results applied: warp -> global RED, as the sweep does per tile
+  const int lane = threadIdx.x & 31;
+  const uint32_t v = warp_result_counts(res, lane);
+  if (v) atomicAdd(&acc[10 + lane], (unsigned long long)v);
 }
 
 __global__ void clear_marks_kernel(uint32_t* marks, const uint2* __restrict__ ops, uint32_t n) {
@@ -1088,12 +1083,9 @@ __global__ void gather_records_kernel(DevCols c, const uint32_t* __restrict__ id
   if (k >= n) return;
   const uint32_t i = idx[k];
   am_record_t r;
-  r.minute = c.minute[i]; r.hour = c.hour[i]; r.dom = c.dom[i]; r.month = c.month[i]; r.dow = c.dow[i];
-  r.finished_at = c.finished_at[i]; r.remedy_finished_at = c.remedy_finished_at[i];
-  r.ras = c.ras[i]; r.flags = c.flags[i];
-  r.runs_limit = c.runs_limit[i]; r.reset_interval = c.reset_interval[i];
-  r.success = c.success[i]; r.failed = c.failed[i]; r.remedy_success = c.remedy_success[i];
-  r.remedy_failed = c.remedy_failed[i]; r.remedy_total = c.remedy_total[i];
+#define AM_LOAD(name) r.name = c.name[i];
+  AM_RECORD_COLUMNS(AM_LOAD)
+#undef AM_LOAD
   r.reserved = 0;
   out[k] = r;
 }

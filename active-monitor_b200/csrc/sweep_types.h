@@ -5,6 +5,7 @@
 #ifndef AMSWEEP_EMULATE  // tests/emu compiles these files for the CPU (cuda_emu.h supplies the model)
 #include <cuda_runtime.h>
 #endif
+#include <stddef.h>
 #include <stdint.h>
 
 #include "../../include/amsweep.h"
@@ -40,12 +41,15 @@
 #endif
 #define AM_SWEEP_KERNEL(closed, masks) sweep_tick_kernel<closed, masks>  // one macro argument
 
+// The sixteen record columns, in am_record_cols_t member order: position = the column id of
+// am_sweep_column_ptr.  am_record_t has a field of the same name and type for each.
+#define AM_RECORD_COLUMNS(X)                                                                        \
+  X(minute) X(hour) X(dom) X(month) X(dow) X(ras) X(flags) X(finished_at) X(runs_limit) X(reset_interval) \
+  X(success) X(failed) X(remedy_success) X(remedy_failed) X(remedy_total) X(remedy_finished_at)
+
 namespace amsweep {
 
-#ifndef AM_BLOCK
-#define AM_BLOCK 256
-#endif
-constexpr int kBlock = AM_BLOCK;
+constexpr int kBlock = 256;
 constexpr int kWarps = kBlock / 32;
 constexpr int kRecPerWarp = 128;             // 2 halves x 32 lanes x 2 records
 constexpr int kTile = kWarps * kRecPerWarp;  // 1024 records per CTA
@@ -61,15 +65,20 @@ constexpr uint32_t kGroupWords = kGroupRecords / 32;     // 256
 constexpr uint32_t kTileWords = kTile / 32;              // 32
 static_assert(kBlock == 256 && kTile == 1024, "bitmap layout: 32 words per tile, 4 per warp");
 
-struct DevCols {
-  uint64_t *minute, *hour, *dom, *month, *dow;
-  int32_t* ras;
-  uint32_t* flags;
-  int64_t* finished_at;
-  int32_t *runs_limit, *reset_interval;
-  int32_t *success, *failed, *remedy_success, *remedy_failed, *remedy_total;
-  int64_t* remedy_finished_at;
-};
+// A shard's device columns are the public column set, passed to kernels by value.  Column k is
+// the k-th pointer of the struct: the host runtime addresses columns by id through that.
+using DevCols = am_record_cols_t;
+constexpr int kNumCols = 16;
+struct ColumnInfo { size_t offset, elem; };
+#define AM_COLUMN_INFO(name) {offsetof(am_record_cols_t, name), sizeof(*am_record_cols_t{}.name)},
+constexpr ColumnInfo kColumns[kNumCols] = {AM_RECORD_COLUMNS(AM_COLUMN_INFO)};
+#undef AM_COLUMN_INFO
+constexpr bool columns_are_a_pointer_array() {
+  for (int k = 0; k < kNumCols; ++k)
+    if (kColumns[k].offset != k * sizeof(void*)) return false;
+  return sizeof(am_record_cols_t) == kNumCols * sizeof(void*);
+}
+static_assert(columns_are_a_pointer_array(), "am_record_cols_t: sixteen pointers in AM_RECORD_COLUMNS order");
 
 // What one tick of one shard leaves behind for the list rebuild (expand_kernel) and for the
 // NVLink exchange: the same four arrays whether they are the sweep's own buffers or the copy
