@@ -141,6 +141,7 @@ SYMBOLS = {
     "am_sweep_tick_device": (C.c_int, [C.c_void_p, i64, u32, C.c_void_p, C.c_void_p, u64,
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "am_sweep_run_ticks": (C.c_int, [C.c_void_p, i64, u64, u32, u64, C.c_void_p]),
+    "am_sweep_run_ticks_view": (C.c_int, [C.c_void_p, i64, u64, u32, u64, C.c_void_p, C.c_void_p]),
     "am_sweep_repeat_after_sec": (C.c_int, [C.c_void_p, i64, u64, u64, C.c_void_p]),
     "am_sweep_next_due": (C.c_int, [C.c_void_p, i64, P(i64)]),
     "am_sweep_read": (C.c_int, [C.c_void_p, u64, u64, C.c_void_p, P(AmRecordCols)]),

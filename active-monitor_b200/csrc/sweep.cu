@@ -171,6 +171,10 @@ struct am_sweep {
   bool early_results = true;  // AMSWEEP_EARLY_RESULTS=0: every posted result is applied inside the sweep
   Staging* pend_clear = nullptr;  // a host tick's drain leaves clear_marks_kernel for after the tick's kernels
   size_t pend_clear_n = 0;
+  // am_sweep_run_ticks_view(AM_SWEEP_BLOCKED): one TickOut per tick of a block, allocated on first use
+  TickRing ring{};
+  uint32_t ring_slots = 0;
+  uint32_t* ring_totals = nullptr;  // [kMaxBlockTicks] pinned + mapped: each slot's emitted count
 };
 
 namespace {
@@ -539,6 +543,183 @@ int reserve_host_out(am_sweep* h, uint64_t entries) {
   return AM_OK;
 }
 
+// Grow the mapped list buffer to hold `entries`, keeping its first `used` entries (a run of ticks
+// appends list after list).  The buffer moves: nothing on the device may still write into it.
+int grow_host_out(am_sweep* h, uint64_t entries, uint64_t used) {
+  if (entries <= h->host_out_entries) return AM_OK;
+  const uint64_t want = (entries + entries / 4 + 4095) / 4096 * 4096;
+  AM_CUDA(h, cudaStreamSynchronize(h->stream));
+  void* np = nullptr;
+  AM_CUDA(h, cudaHostAlloc(&np, want * 5, cudaHostAllocMapped));
+  if (used) {
+    memcpy(np, h->host_out.p, used * 4);
+    memcpy((uint8_t*)np + want * 4, (const uint8_t*)h->host_out.p + h->host_out_entries * 4, used);
+  }
+  h->host_out.release();
+  h->host_out.p = np;
+  h->host_out.cap = want * 5;
+  h->host_out_entries = want;
+  return AM_OK;
+}
+
+void release_ring(am_sweep* h) {
+  TickOut& b = h->ring.base;
+  for (uint32_t* p : {b.bitmap, b.group_count, b.group_prefix, b.tile_exc, b.exc_seg}) if (p) cudaFree(p);
+  b = TickOut{};
+  h->ring_slots = 0;
+}
+
+// The tick ring, `slots` ticks deep, at the strides of the handle's capacity (amsweep.h has the size).
+int reserve_ring(am_sweep* h, uint32_t slots) {
+  if (slots <= h->ring_slots) return AM_OK;
+  AM_CUDA(h, cudaStreamSynchronize(h->stream));
+  release_ring(h);
+  TickRing& r = h->ring;
+  r.tiles = h->cap_padded / kTile;
+  r.groups = (r.tiles + kGroupTiles - 1) / kGroupTiles;
+  r.bitmap_words = r.groups * kGroupWords;
+  r.exc_words = r.tiles * kTile;
+  const int rc = [&]() -> int {
+    if (!h->ring_totals) AM_CUDA(h, cudaHostAlloc((void**)&h->ring_totals, kMaxBlockTicks * 4, cudaHostAllocMapped));
+    const uint64_t words[5] = {r.bitmap_words, r.groups, r.groups + 1, r.tiles, r.exc_words};
+    uint32_t** arrays[5] = {&r.base.bitmap, &r.base.group_count, &r.base.group_prefix, &r.base.tile_exc, &r.base.exc_seg};
+    for (int k = 0; k < 5; ++k) {  // zero: bitmap words past the last CTA are never written; group counts start at 0
+      AM_CUDA(h, cudaMalloc((void**)arrays[k], slots * words[k] * 4));
+      AM_CUDA(h, cudaMemsetAsync(*arrays[k], 0, slots * words[k] * 4, h->stream));
+    }
+    return AM_OK;
+  }();
+  if (rc != AM_OK) {
+    release_ring(h);
+    return rc;
+  }
+  h->ring_slots = slots;
+  return AM_OK;
+}
+
+// am_sweep_run_ticks_view without AM_SWEEP_BLOCKED: one tick after the other, each list expanded into
+// the list buffer behind the previous one, one synchronisation per tick.  start[k]: tick k's first entry.
+int run_lists_ticks(am_sweep* h, int64_t unix_sec0, uint64_t n_ticks, uint32_t mode, am_tick_stats_t* stats,
+                    uint64_t* start) {
+  uint64_t used = 0;
+  for (uint64_t k = 0; k < n_ticks; ++k) {
+    int rc = grow_host_out(h, used + h->n_records, used);
+    if (rc != AM_OK) return rc;
+    ListOut o;
+    if (h->host_out_entries) {
+      void* d = nullptr;
+      AM_CUDA(h, cudaHostGetDevicePointer(&d, h->host_out.p, 0));
+      o.idx = (uint32_t*)d + used;
+      o.act = (uint8_t*)d + h->host_out_entries * 4 + used;
+      o.cap = h->host_out_entries - used;
+    }
+    o.stats = h->d_stats_mapped;
+    rc = launch_tick(h, unix_sec0 + (int64_t)k, mode, o, h->stream);
+    if (rc != AM_OK) return rc;
+    AM_CUDA(h, cudaStreamSynchronize(h->stream));
+    stats[k] = *h->h_stats;
+    stats[k].n_records = h->n_records;
+    start[k] = used;
+    used = (used + stats[k].n_emitted + 3) & ~3ull;  // expand_kernel writes 16-B aligned quads of indices
+  }
+  return AM_OK;
+}
+
+// am_sweep_run_ticks_view with AM_SWEEP_BLOCKED: per block of K ticks, sweep_block_kernel<., true> fills K
+// slots of the tick ring, ring_scan_kernel turns them into offsets and totals, the host waits once and
+// sizes the list buffer, and expand_kernel rebuilds the K lists, up to kMaxWorld ticks per launch.
+// The block length (AMSWEEP_BLOCK_TICKS), the cut at zone-offset changes and the BlockParams are those of the
+// block loop of am_sweep_run_ticks: a change to one belongs in the other.
+int run_lists_blocked(am_sweep* h, int64_t unix_sec0, uint64_t n_ticks, uint32_t mode, am_tick_stats_t* stats,
+                      uint64_t* start) {
+  uint64_t block_ticks = kDefaultBlockTicks;
+  if (const char* e = getenv("AMSWEEP_BLOCK_TICKS")) { long v = atol(e); if (v >= 1 && v <= kMaxBlockTicks) block_ticks = (uint64_t)v; }
+  int rc = reserve_ring(h, (uint32_t)(block_ticks < n_ticks ? block_ticks : n_ticks));
+  if (rc != AM_OK) return rc;
+  am_tick_stats_t* d_stats = nullptr;
+  AM_CUDA(h, cudaMalloc((void**)&d_stats, n_ticks * sizeof(am_tick_stats_t)));
+  struct FreeOnExit {
+    void* p;
+    ~FreeOnExit() { cudaFree(p); }
+  } free_on_exit{d_stats};
+  AM_CUDA(h, cudaMemsetAsync(d_stats, 0, n_ticks * sizeof(am_tick_stats_t), h->stream));
+  uint32_t* d_totals = nullptr;
+  AM_CUDA(h, cudaHostGetDevicePointer((void**)&d_totals, h->ring_totals, 0));
+  const uint32_t n_groups = groups_of(h->n_records), n_tiles = tiles_of(h->n_records);
+  const unsigned grid = (unsigned)((h->n_records + kBlockRecords - 1) / kBlockRecords);
+  uint64_t used = 0;
+  for (uint64_t k = 0; k < n_ticks;) {
+    const int64_t T = unix_sec0 + (int64_t)k;
+    rc = refresh_zones(h, T, h->stream);
+    if (rc != AM_OK) return rc;
+    uint64_t K = n_ticks - k < block_ticks ? n_ticks - k : block_ticks;
+    if (h->tz_n > 1 && h->tz_hi < T + (int64_t)K) K = (uint64_t)(h->tz_hi - T);  // (tz_hi > T after the refresh)
+    BlockParams b{};
+    b.c = h->cols;
+    b.n_records = h->n_records;
+    b.shard_base = h->shard_base;
+    b.seed = h->seed;
+    b.T0 = T;
+    b.K = (uint32_t)K;
+    b.tz_off = h->tz_n > 1 ? (const int32_t*)h->tz_off.p : nullptr;
+    b.stats = reinterpret_cast<unsigned long long*>(d_stats + k);
+    b.ring = h->ring;
+    // exception counts and group counts of the K slots start at zero whatever an earlier call left behind
+    // (ring_scan_kernel re-arms the group counts, but a call that failed in between would not have run it)
+    AM_CUDA(h, cudaMemsetAsync(h->ring.base.tile_exc, 0, K * h->ring.tiles * 4, h->stream));
+    AM_CUDA(h, cudaMemsetAsync(h->ring.base.group_count, 0, K * h->ring.groups * 4, h->stream));
+    if (mode & AM_SWEEP_CLOSED_LOOP) AM_LAUNCH(AM_BLOCK_KERNEL(true, true), grid, kBlockThreads, h->stream, b);
+    else AM_LAUNCH(AM_BLOCK_KERNEL(false, true), grid, kBlockThreads, h->stream, b);
+    AM_LAUNCH(ring_scan_kernel, (unsigned)K, kRingScanThreads, h->stream, h->ring, n_groups, d_totals);
+    h->launches += 2;
+    AM_CUDA(h, cudaGetLastError());
+    AM_CUDA(h, cudaStreamSynchronize(h->stream));
+    // the K lists back to back from `used`; each expand launch starts 16-B aligned
+    uint64_t end = used;
+    for (uint64_t j = 0; j < K; ++j) {
+      if (j % kMaxWorld == 0) end = (end + 3) & ~3ull;
+      start[k + j] = end;
+      end += h->ring_totals[j];
+    }
+    rc = grow_host_out(h, end, used);
+    if (rc != AM_OK) return rc;
+    void* d = nullptr;
+    if (h->host_out.p) AM_CUDA(h, cudaHostGetDevicePointer(&d, h->host_out.p, 0));
+    for (uint64_t j0 = 0; j0 < K; j0 += kMaxWorld) {
+      const uint64_t nj = K - j0 < (uint64_t)kMaxWorld ? K - j0 : (uint64_t)kMaxWorld;
+      const uint64_t s0 = start[k + j0];
+      ExpandParams e{};
+      for (uint64_t j = 0; j < nj; ++j) {
+        const uint64_t t = j0 + j;
+        ExpandSrc& src = e.src[j];
+        src.bitmap = h->ring.base.bitmap + t * h->ring.bitmap_words;
+        src.group_prefix = h->ring.base.group_prefix + t * (h->ring.groups + 1);
+        src.tile_exc = h->ring.base.tile_exc + t * h->ring.tiles;
+        src.exc_seg = h->ring.base.exc_seg + t * h->ring.exc_words;
+        src.base = 0;  // local indices
+        src.n_groups = n_groups;
+        src.n_tiles = n_tiles;
+      }
+      e.out_idx = d ? (void*)((uint32_t*)d + s0) : nullptr;
+      e.out_act = d ? (uint8_t*)d + h->host_out_entries * 4 + s0 : nullptr;
+      e.cap = d ? h->host_out_entries - s0 : 0;
+      e.acc = nullptr;  // the statistics come from the block kernel
+      e.world = (int)nj;
+      e.stats_rank = 0;
+      e.idx_bytes = 4;
+      AM_LAUNCH(expand_kernel, dim3(n_groups, (unsigned)nj), kExpandThreads, h->stream, e);
+      h->launches++;
+    }
+    AM_CUDA(h, cudaGetLastError());
+    used = end;
+    k += K;
+  }
+  AM_CUDA(h, cudaStreamSynchronize(h->stream));
+  AM_CUDA(h, cudaMemcpy(stats, d_stats, n_ticks * sizeof(am_tick_stats_t), cudaMemcpyDeviceToHost));
+  for (uint64_t k = 0; k < n_ticks; ++k) stats[k].n_records = h->n_records;
+  return AM_OK;
+}
+
 // One host tick: drain, four kernels, one synchronisation; the list lands in h->host_out.
 int host_tick(am_sweep* h, int64_t unix_sec, uint32_t mode, am_tick_stats_t* stats) {
   AM_CUDA(h, cudaSetDevice(h->device));
@@ -732,6 +913,8 @@ void am_sweep_destroy(am_sweep_t* h) {
     if (st.drained) cudaEventDestroy(st.drained);
   }
   if (h->marks) cudaFree(h->marks);
+  release_ring(h);
+  if (h->ring_totals) cudaFreeHost(h->ring_totals);
   if (h->h_stats) cudaFreeHost(h->h_stats);
   h->host_out.release();
   h->pin_in.release(); h->dev_in.release();
@@ -1019,6 +1202,7 @@ int am_sweep_run_ticks(am_sweep_t* h, int64_t unix_sec0, uint64_t n_ticks, uint3
     h->last_error = cudaGetErrorString(e);
     rc = AM_E_DEVICE;
   }
+  // (run_lists_blocked repeats this block loop for am_sweep_run_ticks_view: a change here belongs there too.)
   // Temporal blocking (sweep_block.cuh): up to kMaxBlockTicks ticks per pass over the columns.  A block
   // never spans an instant at which a registered zone changes its UTC offset (the kernel holds one
   // offset per zone for the whole block).
@@ -1067,6 +1251,45 @@ int am_sweep_run_ticks(am_sweep_t* h, int64_t unix_sec0, uint64_t n_ticks, uint3
   }
   cudaFree(d_stats);
   return rc;
+}
+
+int am_sweep_run_ticks_view(am_sweep_t* h, int64_t unix_sec0, uint64_t n_ticks, uint32_t mode, uint64_t seed,
+                            am_tick_stats_t* stats_out, am_tick_view_t* views) {
+  if (!h || !stats_out || !views) return AM_E_INVAL;
+  if (n_ticks == 0) return AM_OK;
+  if (n_ticks > (1ull << 24)) return AM_E_INVAL;
+  if (unix_sec0 >= (1ll << 55) - (int64_t)n_ticks || unix_sec0 <= -(1ll << 55)) return AM_E_RANGE;
+  TickGuard g(h);
+  if (!g.ok) return AM_E_BUSY;
+  AM_CUDA(h, cudaSetDevice(h->device));
+  int rc = order_on(h, h->stream);
+  if (rc != AM_OK) return rc;
+  // No tick time: posted results stay pending in the flags, and the first tick's sweep or block kernel
+  // applies and counts them (a block kernel publishes only what it counts itself).
+  rc = drain_staged(h, h->stream);
+  if (rc != AM_OK) return rc;
+  h->seed = seed;
+  h->host_n = 0;  // the list buffer is about to hold a run of lists, no longer the last tick's
+  std::vector<uint64_t> start(n_ticks);
+  AM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
+  if ((mode & AM_SWEEP_BLOCKED) && h->n_records != 0)
+    rc = run_lists_blocked(h, unix_sec0, n_ticks, mode, stats_out, start.data());
+  else
+    rc = run_lists_ticks(h, unix_sec0, n_ticks, mode & ~AM_SWEEP_BLOCKED, stats_out, start.data());
+  if (rc != AM_OK) return rc;
+  AM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
+  AM_CUDA(h, cudaEventSynchronize(h->ev1));
+  float ms = 0;
+  AM_CUDA(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  h->last_ms = ms;
+  const uint8_t* act = h->host_out.p ? (const uint8_t*)h->host_out.p + h->host_out_entries * 4 : nullptr;
+  for (uint64_t k = 0; k < n_ticks; ++k) {
+    views[k].idx_local = h->host_out.p ? (const uint32_t*)h->host_out.p + start[k] : nullptr;
+    views[k].action = act ? act + start[k] : nullptr;
+    views[k].n = stats_out[k].n_emitted;
+    views[k].shard_base = h->shard_base;
+  }
+  return AM_OK;
 }
 
 static int read_impl(am_sweep_t* h, uint64_t first, uint64_t n, const uint64_t* idx, am_record_cols_t* out);

@@ -21,10 +21,17 @@
 // complete_closed_loop — so the per-tick statistics and the
 // columns after the block are bit-identical to K single ticks (tests: run_ticks blocked == unblocked ==
 // oracle).  Work is O(events), not O(records x ticks); the columns are read and written once per K
-// ticks.  What it does NOT produce is the per-tick (index, action) lists: a run of ticks publishes
-// per-tick statistics (counts, action counts, index checksums — am_tick_stats_t), which is all
-// am_sweep_run_ticks ever returned to the host.  Reported separately from the K = 1 roofline number.
+// ticks.  Reported separately from the K = 1 roofline number.
+//
+// am_sweep_run_ticks wants per-tick statistics only (am_tick_stats_t): sweep_block_kernel<CLOSED, false>.
+// am_sweep_run_ticks_view also wants every tick's (index, action) list: sweep_block_kernel<CLOSED, true>
+// additionally leaves, per tick of the block, exactly what sweep_tick_kernel leaves for one tick — an
+// emitted bitmap, per-group counts and per-tile exception segments (TickOut) — in slot t of a TickRing.
+// ring_scan_kernel turns the counts into offsets for all K slots at once, and the unchanged expand_kernel
+// rebuilds up to 16 ticks' lists per launch (its "ranks" are the ticks; its output, their concatenation).
 #pragma once
+
+#include <type_traits>
 
 namespace amsweep {
 
@@ -38,6 +45,19 @@ constexpr int kBlockThreads = 128;
 constexpr int kBlockMinCtas = 8;
 constexpr int kBlockRecords = 4 * kBlockThreads;  // four consecutive records per thread in the classification pass
 constexpr int kBlockClasses = 4;                  // by expected number of events in the block: <= 2, <= 8, <= 24, more
+constexpr int kBlockWords = kBlockRecords / 32;   // emitted-bitmap words of one CTA per tick
+static_assert(kTile == 2 * kBlockRecords && kGroupRecords % kBlockRecords == 0, "a tile is two block CTAs");
+
+// K TickOut slots back to back, one per tick of a block (am_sweep_run_ticks_view with AM_SWEEP_BLOCKED).
+// Slot t of each array starts at t * (its per-slot stride); the strides are those of the handle's
+// capacity, so every slot has the layout expand_kernel reads.
+struct TickRing {
+  TickOut base;           // slot 0
+  uint64_t bitmap_words;  // per-slot strides, in u32 elements: n_groups * 256
+  uint64_t groups;        // group_count; group_prefix has groups + 1 per slot
+  uint64_t tiles;         // tile_exc
+  uint64_t exc_words;     // exc_seg: tiles * 1024
+};
 
 struct BlockParams {
   DevCols c;
@@ -46,6 +66,7 @@ struct BlockParams {
   uint32_t K;                  // ticks in the block, <= kMaxBlockTicks
   const int32_t* tz_off;       // per-zone UTC offsets valid for the whole block (NULL: no zone registered)
   unsigned long long* stats;   // K rows of 16 accumulators (am_tick_stats_t layout), zero on entry
+  TickRing ring;               // sweep_block_kernel<., true> only: tile_exc and group_count zero on entry
 };
 
 // first tick index u > t at which the LOCAL second (UTC + off) is 0
@@ -68,17 +89,46 @@ struct BlockStats {
   uint32_t n_list[kBlockClasses];
 };
 
-__device__ __forceinline__ void block_constant(BlockStats& S, int which, int64_t t_from, int64_t K, uint64_t g, uint32_t loc) {
+// What the lists add: 8 768 B (static shared memory 25 168 B instead of 16 400; with the 1 KB reserved per CTA,
+// 26 192 B instead of 17 424: still 8 CTAs per SM).  Still 64 registers; the spills grow to 16 B (closed loop)
+// and 28 B stored / 60 B loaded (open loop), from 4 and 12 B without the lists (ptxas, CUDA 12.9).
+struct BlockLists {
+  uint32_t emit[kMaxBlockTicks][kBlockWords];  // records of the CTA with an event action at tick t
+  uint32_t c_parse[kBlockWords];               // constant emitter of PARSE_ERROR (else of SUBMIT_HC)
+  uint8_t c_from[kBlockRecords];               // first tick of the record's constant action; 0xFF: none
+};
+struct BlockStatsLists : BlockStats {
+  BlockLists lists;
+};
+
+// (record loc of the CTA at cta_base, tick t) emits `act`, which is not a bare SUBMIT_HC: an entry of
+// the tile's exception segment in slot t.  Two CTAs share a tile; expand_kernel finds an entry's place
+// from its offset, so their order within the segment does not matter.
+__device__ __forceinline__ void ring_exception(const TickRing& r, int64_t t, uint64_t cta_base, uint32_t loc, uint32_t act) {
+  const uint64_t tile = cta_base / kTile;
+  const uint32_t off = (uint32_t)(cta_base % kTile) + loc;
+  const uint32_t pos = atomicAdd(r.base.tile_exc + (uint64_t)t * r.tiles + tile, 1u);
+  r.base.exc_seg[(uint64_t)t * r.exc_words + tile * kTile + pos] = (off << 8) | act;
+}
+
+template <bool LISTS = false>
+__device__ __forceinline__ void block_constant(BlockStats& S, int which, int64_t t_from, int64_t K, uint64_t g, uint32_t loc,
+                                               BlockLists* L = nullptr) {
   if (t_from >= K) return;
   atomicAdd(&S.c_cnt[t_from][which], 1u);
   atomicAdd(&S.c_sum[t_from][which], loc);
   atomicXor(&S.c_x[t_from][which][0], (uint32_t)g);
   atomicXor(&S.c_x[t_from][which][1], (uint32_t)(g >> 32));
+  if constexpr (LISTS) {  // (a record becomes a constant emitter at most once)
+    L->c_from[loc] = (uint8_t)t_from;
+    if (which) atomicOr(&L->c_parse[loc >> 5], 1u << (loc & 31u));
+  }
 }
 
 // One record through the block, event by event (see the header of this file).
-template <bool CLOSED>
-__device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S, uint64_t cta_base, uint32_t loc) {
+template <bool CLOSED, bool LISTS = false>
+__device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S, uint64_t cta_base, uint32_t loc,
+                                             BlockLists* L = nullptr) {
   constexpr uint32_t kPend = AM_F_PENDING_OK | AM_F_PENDING_FAIL | AM_F_REMEDY_PENDING;
   const int64_t K = (int64_t)p.K;
   const uint64_t i = cta_base + loc;
@@ -170,6 +220,10 @@ __device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S
       atomicXor(&S.x[t][0], (uint32_t)g);
       atomicXor(&S.x[t][1], (uint32_t)(g >> 32));
       atomicAdd(&S.sum[t], loc);
+      if constexpr (LISTS) {
+        atomicOr(&L->emit[t][loc >> 5], 1u << (loc & 31u));
+        if (act != AM_ACT_SUBMIT_HC) ring_exception(p.ring, t, cta_base, loc, act);
+      }
     }
     if (res) {
 #pragma unroll
@@ -177,8 +231,8 @@ __device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S
         if ((res >> (8 * q)) & 0xFFu) atomicAdd(&S.cnt[t][9 + q], (res >> (8 * q)) & 0xFFu);
     }
     // from here on the same bare action on every tick, and nothing changes any more?
-    if (kind == AM_KIND_PARSE_ERROR) { block_constant(S, 1, t + 1, K, g, loc); break; }
-    if (!CLOSED && is_iv && due) { block_constant(S, 0, t + 1, K, g, loc); break; }  // stays due: nothing completes it in open loop
+    if (kind == AM_KIND_PARSE_ERROR) { block_constant<LISTS>(S, 1, t + 1, K, g, loc, L); break; }
+    if (!CLOSED && is_iv && due) { block_constant<LISTS>(S, 0, t + 1, K, g, loc, L); break; }  // stays due: nothing completes it in open loop
     t = next_event(t);
   }
 
@@ -195,15 +249,22 @@ __device__ __forceinline__ void block_record(const BlockParams& p, BlockStats& S
   }
 }
 
-template <bool CLOSED>
+template <bool CLOSED, bool LISTS = false>
 __global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kernel(const BlockParams p) {
-  __shared__ BlockStats S;
+  __shared__ typename std::conditional<LISTS, BlockStatsLists, BlockStats>::type S;
+  BlockLists* L = nullptr;
   const int tid = threadIdx.x;
   {
     uint32_t* z = reinterpret_cast<uint32_t*>(&S);
     constexpr int kZero = (int)(offsetof(BlockStats, list) / 4);  // everything before the lists
     for (int k = tid; k < kZero; k += kBlockThreads) z[k] = 0;
     if (tid < kBlockClasses) S.n_list[tid] = 0;
+  }
+  if constexpr (LISTS) {
+    L = &S.lists;
+    for (uint32_t k = (uint32_t)tid; k < p.K * kBlockWords; k += kBlockThreads) (&L->emit[0][0])[k] = 0;
+    if (tid < kBlockWords) L->c_parse[tid] = 0;
+    reinterpret_cast<uint32_t*>(L->c_from)[tid] = 0xFFFFFFFFu;  // (kBlockRecords = 4 x kBlockThreads)
   }
   __syncthreads();
 
@@ -236,7 +297,7 @@ __global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kern
       const uint64_t g = p.shard_base + cta_base + loc;
       int64_t n_ev = 0;  // expected events in the block (an upper bound is fine: it only picks the list)
       if (kind == AM_KIND_PARSE_ERROR) {
-        if (!first_tick) { block_constant(S, 1, 0, K, g, loc); continue; }
+        if (!first_tick) { block_constant<LISTS>(S, 1, 0, K, g, loc, L); continue; }
         n_ev = 1;
       } else if (kind == AM_KIND_STOPPED) {
         n_ev = (first_tick || !(f & AM_F_STOPPED_REPORTED)) ? 1 : 0;
@@ -249,13 +310,13 @@ __global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kern
       } else {  // INTERVAL / CRON_EVERY
         const int64_t step = rasv > 0 ? (int64_t)rasv : 1;
         if (!(f & AM_F_TIMER_ARMED) || first_tick) {
-          if (!CLOSED && !first_tick) { block_constant(S, 0, 0, K, g, loc); continue; }  // due on every tick, nothing changes
+          if (!CLOSED && !first_tick) { block_constant<LISTS>(S, 0, 0, K, g, loc, L); continue; }  // due on every tick, nothing changes
           n_ev = 1 + (K - 1) / step;
         } else {
           int64_t d = fa + (int64_t)rasv - p.T0;
           if (d < 0) d = 0;
           if (d >= K) continue;  // its timer fires after the block
-          if (!CLOSED) { block_constant(S, 0, d, K, g, loc); continue; }  // due from tick d on
+          if (!CLOSED) { block_constant<LISTS>(S, 0, d, K, g, loc, L); continue; }  // due from tick d on
           n_ev = 1 + (K - 1 - d) / step;
         }
       }
@@ -276,7 +337,7 @@ __global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kern
   for (int c = kBlockClasses - 1; c >= 0; --c) {
     const uint32_t n = S.n_list[c];
     for (uint32_t k = ((uint32_t)tid + (uint32_t)(kBlockThreads / 4) * (uint32_t)c) & (kBlockThreads - 1); k < n; k += kBlockThreads)
-      block_record<CLOSED>(p, S, cta_base, S.list[c][k]);
+      block_record<CLOSED, LISTS>(p, S, cta_base, S.list[c][k], L);
   }
   __syncthreads();
 
@@ -313,6 +374,74 @@ __global__ void __launch_bounds__(kBlockThreads, kBlockMinCtas) sweep_block_kern
       const uint32_t cnt = S.cnt[t][0];
       if (cnt) atomicAdd(dst, (unsigned long long)cnt * gbase + S.sum[t]);
     }
+  }
+
+  if constexpr (LISTS) {
+    // ---- the constant emitters join the bitmap of every tick from their first one on: warp w owns words
+    //      w, w + 4, ... (one ballot per word and tick); a parse error is an exception on each of them
+    const uint32_t lane = (uint32_t)tid & 31u;
+    for (int w = tid >> 5; w < kBlockWords; w += kBlockThreads / 32) {
+      const uint32_t loc = 32u * (uint32_t)w + lane;
+      const uint32_t from = L->c_from[loc];
+      const bool parse = ((L->c_parse[w] >> lane) & 1u) != 0;
+      if (!__any_sync(kFull, from != 0xFFu)) continue;  // (warp-uniform)
+      for (uint32_t t = 0; t < p.K; ++t) {
+        const bool on = from <= t;
+        const uint32_t m = __ballot_sync(kFull, on);
+        if (lane == 0) L->emit[t][w] |= m;
+        if (on && parse) ring_exception(p.ring, t, cta_base, loc, AM_ACT_PARSE_ERROR);
+      }
+    }
+    __syncthreads();
+    // ---- slot t: this CTA's 16 bitmap words (64 B), and its emitted count into the group's counter
+    const uint64_t word0 = cta_base / 32, group = cta_base / kGroupRecords;
+    for (uint32_t k = (uint32_t)tid; k < p.K * kBlockWords; k += kBlockThreads) {
+      const uint32_t t = k / kBlockWords, w = k % kBlockWords;
+      p.ring.base.bitmap[(uint64_t)t * p.ring.bitmap_words + word0 + w] = L->emit[t][w];
+    }
+    for (uint32_t t = (uint32_t)tid; t < p.K; t += kBlockThreads)
+      if (S.cnt[t][0]) atomicAdd(p.ring.base.group_count + (uint64_t)t * p.ring.groups + group, S.cnt[t][0]);
+  }
+}
+
+// Per-slot group offsets of a tick ring: one CTA per tick, the scan of scan_groups_kernel over that
+// slot's group counts.  Re-arms the counts and writes each tick's total to totals[t] (mapped host
+// memory: the host sizes its list buffer from them before expand_kernel runs).
+constexpr int kRingScanThreads = 256;
+__global__ void __launch_bounds__(kRingScanThreads) ring_scan_kernel(const TickRing r, uint32_t n_groups, uint32_t* totals) {
+  __shared__ uint32_t s_warp[kRingScanThreads / 32];
+  __shared__ uint32_t s_carry;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint64_t t = blockIdx.x;
+  uint32_t* count = r.base.group_count + t * r.groups;
+  uint32_t* prefix = r.base.group_prefix + t * (r.groups + 1);
+  if (tid == 0) s_carry = 0;
+  __syncthreads();
+  for (uint32_t g0 = 0; g0 < n_groups; g0 += kRingScanThreads) {
+    const uint32_t g = g0 + (uint32_t)tid;
+    const uint32_t c = g < n_groups ? count[g] : 0u;
+    uint32_t incl = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t up = __shfl_up_sync(kFull, incl, d);
+      if (lane >= d) incl += up;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    uint32_t before = s_carry;
+    for (int k = 0; k < warp; ++k) before += s_warp[k];
+    const uint32_t excl = before + incl - c;
+    if (g < n_groups) {
+      prefix[g] = excl;
+      count[g] = 0;
+    }
+    __syncthreads();  // every thread has read s_carry / s_warp of this round
+    if (tid == kRingScanThreads - 1) s_carry = excl + c;
+    __syncthreads();
+  }
+  if (tid == 0) {
+    prefix[n_groups] = s_carry;
+    totals[t] = s_carry;
   }
 }
 

@@ -40,6 +40,7 @@
 #endif
 #endif
 #define AM_SWEEP_KERNEL(closed, masks) sweep_tick_kernel<closed, masks>  // one macro argument
+#define AM_BLOCK_KERNEL(closed, lists) sweep_block_kernel<closed, lists>
 
 // The sixteen record columns, in am_record_cols_t member order: position = the column id of
 // am_sweep_column_ptr.  am_record_t has a field of the same name and type for each.

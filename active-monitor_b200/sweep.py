@@ -293,6 +293,24 @@ class Sweep:
                                                  out.ctypes.data), "am_sweep_run_ticks")
         return out
 
+    def run_ticks_view(self, unix_sec0: int, n_ticks: int, mode: int = 0, seed: int = 0):
+        """run_ticks with every tick's list: (stats, [(u32 LOCAL idx view, u8 action view), ...]).
+        The arrays alias the library's pinned buffer: valid until the next tick or run on the handle."""
+        out = np.zeros(n_ticks, dtype=L.STATS_DTYPE)
+        views = (L.AmTickView * max(n_ticks, 1))()
+        self._check(self._lib.am_sweep_run_ticks_view(self._h, unix_sec0, n_ticks, mode, seed,
+                                                      out.ctypes.data, views), "am_sweep_run_ticks_view")
+        lists = []
+        for v in views[:n_ticks]:
+            n = int(v.n)
+            if n == 0:
+                lists.append((np.empty(0, np.uint32), np.empty(0, np.uint8)))
+                continue
+            idx = np.ctypeslib.as_array(C.cast(v.idx_local, C.POINTER(C.c_uint32)), shape=(n,))
+            act = np.ctypeslib.as_array(C.cast(v.action, C.POINTER(C.c_uint8)), shape=(n,))
+            lists.append((idx, act))
+        return out, lists
+
     def repeat_after_sec(self, unix_sec: int, first: int, n: int) -> np.ndarray:
         """hcc.go:262 for every record of [first, first+n): Next() evaluated on the device."""
         out = np.zeros(n, dtype=np.int64)

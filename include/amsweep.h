@@ -233,12 +233,13 @@ typedef struct am_tick_stats {
                                      with its preset outcome (SURVEY B.3)     */
 #define AM_SWEEP_FULL_SCAN 0x2u   /* read every schedule column even on ticks
                                      where no 5-field cron can fire (sec!=0)  */
-#define AM_SWEEP_BLOCKED 0x4u     /* am_sweep_run_ticks only: temporal blocking.  Blocks of consecutive
+#define AM_SWEEP_BLOCKED 0x4u     /* am_sweep_run_ticks(_view) only: temporal blocking.  Blocks of consecutive
                                      ticks (96; AMSWEEP_BLOCK_TICKS, at most 128) are evaluated in one pass over the columns,
                                      every record stepped from event to event (its next repeat timer,
                                      hcc.go:751; its next cron minute) — per-tick statistics and the
-                                     columns afterwards are identical to tick-by-tick evaluation, but
-                                     no per-tick lists are produced                                */
+                                     columns afterwards are identical to tick-by-tick evaluation.
+                                     am_sweep_run_ticks returns statistics only; the per-tick lists
+                                     of a blocked run come from am_sweep_run_ticks_view            */
 
 /* One shard of the record array on one CUDA device.  `capacity` slots are
  * allocated up front; `shard_base` is added to local indices wherever a
@@ -331,10 +332,28 @@ int am_sweep_tick_shard(am_sweep_t*, int64_t unix_sec, uint32_t mode, void* cuda
 /* Streaming: n_ticks consecutive one-second ticks starting at unix_sec0,
  * back-to-back on the device (BASELINE config 5).  Per-tick stats are written
  * to stats_out[0..n_ticks) (host).  Emitted lists go to an HBM ring and are
- * not copied to the host (with AM_SWEEP_BLOCKED there are none: see above).
+ * not copied to the host (with AM_SWEEP_BLOCKED there are none); am_sweep_run_ticks_view
+ * returns them.
  * `seed` keys the closed-loop outcome sequence. */
 int am_sweep_run_ticks(am_sweep_t*, int64_t unix_sec0, uint64_t n_ticks, uint32_t mode,
                        uint64_t seed, am_tick_stats_t* stats_out);
+
+/* am_sweep_run_ticks, and in addition the ascending (local index, action) list of every tick.
+ * views[k] (k < n_ticks) describes tick unix_sec0 + k, in the form am_sweep_tick_view returns.
+ * All lists live back to back in the library's pinned host buffer (each one or each group of up to
+ * 16 starts on a multiple of 4 entries). That buffer grows to hold the whole run at 5 B per entry,
+ * so choose n_ticks to match. The views stay valid until the next am_sweep_tick* /
+ * am_sweep_run_ticks* call on the handle; am_sweep_last_list finds no list after this call.
+ * Works with and without AM_SWEEP_BLOCKED / AM_SWEEP_CLOSED_LOOP. Both forms return identical lists,
+ * statistics and columns, and these are identical to n_ticks calls of am_sweep_tick. Staged results
+ * are applied, and counted, at the first tick.
+ * Without AM_SWEEP_BLOCKED the ticks run one after the other, one synchronisation each. With it, a
+ * block of K ticks (AMSWEEP_BLOCK_TICKS, 96 by default) costs one synchronisation: the block kernel
+ * leaves each tick's emitted set in a device "tick ring" of K slots, allocated on the first blocked
+ * call and kept until am_sweep_destroy: K x (4.13 B x capacity) of device memory, about 3.9 GB for
+ * 10 M records at K = 96 (5.3 GB at K = 128). */
+int am_sweep_run_ticks_view(am_sweep_t*, int64_t unix_sec0, uint64_t n_ticks, uint32_t mode,
+                            uint64_t seed, am_tick_stats_t* stats_out, am_tick_view_t* views);
 
 /* RepeatAfterSec of records [first, first+n) as the reference derives it at
  * reconcile time (hcc.go:259-262): Next(unix_sec) - unix_sec for a 5-field

@@ -35,6 +35,13 @@ ap.add_argument("--compare-unblocked", action="store_true", help="with --blocked
 ap.add_argument("--per-tick", type=int, default=0,
                 help="also time this many ticks one by one (CUDA events around the three kernels of "
                      "each tick) and report p50 / p99 / max per-tick device time")
+ap.add_argument("--lists", action="store_true", help="time am_sweep_run_ticks_view (every tick's list to host memory), "
+                "blocked and unblocked, against am_sweep_run_ticks(BLOCKED) without lists, over --windows windows of "
+                "--window ticks; compare the lists of the two forms and, on the first --sub records, with the oracle")
+ap.add_argument("--window", type=int, default=960, help="with --lists: ticks per call")
+ap.add_argument("--windows", type=int, default=2, help="with --lists: consecutive calls (the first one allocates; "
+                "86400 / 960 = 90 is the whole day)")
+ap.add_argument("--profile-dir", default="", help="with --lists: write the torch.profiler kernel table here")
 a = ap.parse_args()
 
 am = importlib.import_module("active-monitor_b200")
@@ -44,6 +51,107 @@ mode = am.SWEEP_CLOSED_LOOP | (am.SWEEP_FULL_SCAN if a.full_scan else 0) | (am.S
 fields = am.abi.STAT_FIELDS
 
 cols = amgen.fill(a.config, seed, 0, a.n, T0, lib.am_healthcheck_classify)
+
+
+def gpu_name_and_power_limit():
+    import subprocess
+    try:
+        return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                              capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+    except Exception as e:  # (reported, never guessed)
+        return f"unknown ({e})"
+
+
+def lists_run():
+    """--lists: what the per-tick lists cost, and that both forms return the same lists."""
+    W, nw = a.window, a.windows
+    blocked, plain = mode | am.SWEEP_BLOCKED, mode & ~am.SWEEP_BLOCKED
+    with am.Sweep(capacity=1000) as w:  # load the modules of every kernel once
+        w.load_range(0, {k: np.ascontiguousarray(v[:1000]) for k, v in cols.items()})
+        for m in (blocked, plain):
+            w.run_ticks_view(T0, 4, m, seed)
+        w.run_ticks(T0, 4, blocked, seed)
+    out = {"gpu": gpu_name_and_power_limit(), "window_ticks": W, "windows": nw, "per_window": []}
+    hb, hu, hn = am.Sweep(capacity=a.n), am.Sweep(capacity=a.n), am.Sweep(capacity=a.n)
+    identical = True
+    for h in (hb, hu, hn):
+        h.load_range(0, cols)
+    for k in range(nw):
+        t = T0 + k * W
+        row = {"first_tick": t}
+        t0 = time.perf_counter()
+        sb, lb = hb.run_ticks_view(t, W, blocked, seed)
+        row["blocked_lists_us_per_tick"] = (time.perf_counter() - t0) * 1e6 / W
+        t0 = time.perf_counter()
+        su, lu = hu.run_ticks_view(t, W, plain, seed)
+        row["unblocked_lists_us_per_tick"] = (time.perf_counter() - t0) * 1e6 / W
+        t0 = time.perf_counter()
+        sn = hn.run_ticks(t, W, blocked, seed)
+        row["blocked_no_lists_us_per_tick"] = (time.perf_counter() - t0) * 1e6 / W
+        row["blocked_no_lists_device_us_per_tick"] = hn.last_kernel_ms * 1e3 / W
+        same = all(np.array_equal(sb[f], su[f]) and np.array_equal(sb[f], sn[f]) for f in fields)
+        same &= all(np.array_equal(bi, ui) and np.array_equal(ba, ua) for (bi, ba), (ui, ua) in zip(lb, lu))
+        identical &= bool(same)
+        n_ent = np.array([len(i) for i, _ in lb], dtype=np.float64)
+        row["entries_per_tick_mean"] = float(n_ent.mean())
+        row["entries_per_tick_max"] = int(n_ent.max())
+        row["host_bytes_per_tick_mean"] = float(n_ent.mean() * 5)
+        out["per_window"].append(row)
+    out["lists_identical"] = identical
+    out["columns_identical"] = bool(all(np.array_equal(x, y) and np.array_equal(x, z) for x, y, z in
+                                        ((hb.read_range(0, a.n)[c], hu.read_range(0, a.n)[c], hn.read_range(0, a.n)[c])
+                                         for c in am.COLUMN_NAMES)))
+    for h in (hb, hu, hn):
+        h.close()
+    # the split of one steady-state window: kernel time by kernel from torch.profiler (CUPTI), in a run of its own
+    if a.profile_dir:
+        import torch
+        from torch.profiler import ProfilerActivity, profile
+        torch.cuda.init()
+        with am.Sweep(capacity=a.n) as hp:
+            hp.load_range(0, cols)
+            hp.run_ticks_view(T0, W, blocked, seed)  # allocations
+            with profile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
+                t0 = time.perf_counter()
+                hp.run_ticks_view(T0 + W, W, blocked, seed)
+                wall = time.perf_counter() - t0
+        split = {}
+        for ev in prof.key_averages():
+            us = getattr(ev, "device_time_total", 0) or getattr(ev, "cuda_time_total", 0)
+            for key in ("sweep_block_kernel", "ring_scan_kernel", "expand_kernel", "Memset"):
+                if key in ev.key and us:
+                    split[key] = split.get(key, 0.0) + us / W
+        busy = sum(split.values())
+        out["split_us_per_tick"] = dict(split, wall=wall * 1e6 / W, host_and_synchronisation=wall * 1e6 / W - busy)
+        os.makedirs(a.profile_dir, exist_ok=True)
+        with open(os.path.join(a.profile_dir, "run_ticks_view_kernels.txt"), "w") as f:
+            f.write(prof.key_averages().table(sort_by="self_device_time_total" if hasattr(prof.key_averages()[0], "self_device_time_total") else "self_cuda_time_total", row_limit=30))
+    # the oracle's lists on the first --sub records, both forms
+    if a.sub:
+        sub = {k: np.ascontiguousarray(v[: a.sub]) for k, v in cols.items()}
+        osub = amgen.fill(a.config, seed, 0, a.sub, T0, oracle_c.load().orc_classify)
+        got = {}
+        for m in (blocked, plain):
+            with am.Sweep(capacity=a.sub) as h:
+                h.load_range(0, sub)
+                st, li = h.run_ticks_view(T0, W, m, seed)
+                got[m] = (st, [(i.copy(), x.copy()) for i, x in li])
+        ok = True
+        for k in range(W):
+            wi, wa, ws = oracle_c.sweep(osub, T0 + k, mode=1, seed=seed)
+            for m in (blocked, plain):
+                st, li = got[m]
+                ok &= all(int(st[f][k]) == ws[f] for f in fields)
+                ok &= np.array_equal(li[k][0].astype(np.uint64), wi) and np.array_equal(li[k][1].astype(np.uint32), wa)
+        out["oracle_lists_equal"] = {"records": a.sub, "ticks": W, "ok": bool(ok)}
+    out["workload"] = (f"config {a.config}: {a.n} records, closed loop, seed 5, {nw} x {W} one-second ticks from "
+                       "2026-09-21T00:00:00Z; times are host clocks around each call (every call ends synchronised)")
+    return out
+
+
+if a.lists:
+    print(json.dumps(lists_run()))
+    sys.exit(0)
 with am.Sweep(capacity=a.n) as s:
     s.load_range(0, cols)
     t0 = time.perf_counter()
